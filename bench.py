@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — env-steps/s of the batched PCT step (BASELINE.json metric) on N B200s of one node.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--setting S] [--envs-per-gpu E] [--continuous]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl ours|reference] [--setting S] [--envs-per-gpu E] [--continuous] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 A "step" is ONE batched environment step over all envs of a rank: the synthetic uniform-valid-leaf policy kernel + the PCT step
@@ -20,6 +20,8 @@ The same JSON line carries the other BASELINE configs as sub-records under `conf
 `vec_env`  : the same metric through the reference-facing VecEnv surface (PctVecEnv.step: device observation, host reward / done / infos).
 `roofline` : HBM roofline of the dominant kernel group, algorithmic bytes per launch (DESIGN.md section 5) / its mean duration measured here
              with CUDA events (second pass with events between the kernels).
+`--dump-outputs DIR`: after the timed steps, what the last timed step of the headline returned (rank 0) is written as DIR/<name>.npy, so
+             that two builds can be compared output for output on identical seeded inputs (see dump_outputs).
 `cpu_baseline` / `--impl reference`: the CPU restatement of the reference env (oracle/, C, pthreads over envs like the reference's
              ShmemVecEnv workers) on this box's host cores; >= 3 repeats of >= 1 s each, median reported (min / max beside it).
 """
@@ -38,6 +40,7 @@ ITEM_SET = [(i, j, k) for i in range(1, 6) for j in range(1, 6) for k in range(1
 ITEM_SEED, POLICY_SEED = 1234, 4321
 METRIC = "env-steps/s (batched PCT step)"
 PREROLL = 256  # steps after the synchronised reset before anything is timed: the batch reaches its steady-state episode mix
+DUMP_LIMIT = 63 * 10 ** 6  # array bytes written by --dump-outputs at most: under 64 MB with the .npy headers
 
 
 def parse():
@@ -54,7 +57,11 @@ def parse():
     ap.add_argument("--skip-configs", action="store_true", help="headline only: no sub-records for the other BASELINE configs")
     ap.add_argument("--continuous", action="store_true", help="BASELINE config 4: PctContinuous, sample_from_distribution, bin 1x1x1")
     ap.add_argument("--preroll", type=int, default=PREROLL)
-    return ap.parse_args()
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write what the last timed step returned as DIR/<name>.npy (--impl ours)")
+    a = ap.parse_args()
+    if a.dump_outputs and a.impl != "ours":
+        ap.error("--dump-outputs needs --impl ours")
+    return a
 
 
 def workload_name(setting, continuous, envs_per_gpu, n_gpus):
@@ -194,10 +201,11 @@ def make_batch(setting, continuous, n, rank, local):
     return pct_b200.PctBatch(n, setting, item_set=ITEM_SET, seed=ITEM_SEED, env_id_base=rank * n, device=local)
 
 
-def measure(cx, setting, continuous, n, K, W, preroll, kernels=True, keep=False):
+def measure(cx, setting, continuous, n, K, W, preroll, kernels=True, keep=False, last=None):
     """Device-timed throughput of one configuration on this rank's GPU (all ranks call it together): reset, `preroll` + W untimed steps,
     K timed steps (CUDA events per step, L2 flushed before each, barrier on both sides), then — discrete only — a second pass of K steps
-    with events between the kernels for the per-kernel durations."""
+    with events between the kernels for the per-kernel durations.  If `last` is a dict, it receives copies of what the last timed step
+    returned (leaf indices of the policy kernel, observation, reward, done, info), taken before the second pass overwrites them."""
     import torch
     batch = make_batch(setting, continuous, n, cx.rank, cx.local)
     batch.reset()
@@ -216,13 +224,15 @@ def measure(cx, setting, continuous, n, K, W, preroll, kernels=True, keep=False)
         ev[t][0].record()
         idx = batch.random_policy(POLICY_SEED, T0 + t)
         ev[t][1].record()
-        _, _, _, info = batch.step(leaf_idx=idx)
+        obs, rew, done, info = batch.step(leaf_idx=idx)
         ev[t][2].record()
         if t % 16 == 0:
             stats += torch.stack([info[:, 0].double().mean(), info[:, 5].double().mean(), info[:, 6].double().mean(), info[:, 7].double().mean()])
     cx.barrier()
     wall = time.perf_counter() - t_wall0
     launches = batch.kernel_launches - l0
+    if last is not None:
+        last.update(zip(("leaf_idx", "obs", "reward", "done", "info"), (x.clone() for x in (idx, obs, rew, done, info))))
     kms, ksteps = {}, 0
     if kernels and not continuous:
         batch.profile(True)
@@ -311,6 +321,25 @@ def roofline_of(rec, setting, continuous, n, obs_len, delta_obs):
     return out
 
 
+def dump_outputs(dirname, last):
+    """Writes the arrays of `last` (see measure) as DIR/<name>.npy: observation and reward in float32 as returned, done in float32, leaf
+    indices and the raw int32 info records (include/pct_b200.h pct_step_info) in float64, both exact.  If they exceed DUMP_LIMIT, the
+    same fixed seeded sample of envs is taken from each, and its env indices are written as env_index.npy."""
+    import numpy as np
+    arrays = {"leaf_idx": last["leaf_idx"].cpu().numpy().astype(np.float64), "obs": last["obs"].float().cpu().numpy(),
+              "reward": last["reward"].float().cpu().numpy(), "done": last["done"].cpu().numpy().astype(np.float32),
+              "info": last["info"].cpu().numpy().astype(np.float64)}
+    n = len(arrays["obs"])
+    total = sum(v.nbytes for v in arrays.values())
+    if total > DUMP_LIMIT:
+        rows = np.sort(np.random.default_rng(0).choice(n, n * DUMP_LIMIT // (total + 8 * n), replace=False))
+        arrays = {k: v[rows] for k, v in arrays.items()}
+        arrays["env_index"] = rows.astype(np.float64)
+    os.makedirs(dirname, exist_ok=True)
+    for k, v in arrays.items():
+        np.save(os.path.join(dirname, k + ".npy"), v)
+
+
 def run_ours(a):
     import numpy as np
     import torch
@@ -346,8 +375,11 @@ def run_ours(a):
     if sampler:
         sampler.start()
         time.sleep(0.3)
-    head, batch = measure(cx, a.setting, a.continuous, n, K, W, a.preroll, keep=True)
+    last = {} if a.dump_outputs and rank == 0 else None
+    head, batch = measure(cx, a.setting, a.continuous, n, K, W, a.preroll, keep=True, last=last)
     clocks = sampler.finish() if sampler else None
+    if last:
+        dump_outputs(a.dump_outputs, last)
     ol = batch.obs_len
 
     # ---- e2e: host buffers through pct_step_host, host policy on the returned records ----

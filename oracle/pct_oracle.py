@@ -102,6 +102,7 @@ class OracleDiscrete(object):
         self.L.pcto_set_random_items(self.h, _dp(self._items), len(self._items), int(seed), int(gid))
 
     def set_trajectory_length(self, n):
+        self.L.pcto_set_trajectory_length.argtypes = [C.c_void_p, C.c_int]
         self.L.pcto_set_trajectory_length(self.h, int(n))
 
     def reset(self):

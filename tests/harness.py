@@ -1,4 +1,6 @@
 """Shared helpers for the parity tests (test infrastructure)."""
+import hashlib
+
 import numpy as np
 
 from pct_oracle import OracleDiscrete, policy_pick, rnd_u64  # noqa: F401  (oracle/ is on sys.path via conftest)
@@ -15,6 +17,17 @@ def make_stream(seed, env, n, setting):
         s[d, :3] = ITEM_SET[rnd_u64(seed, env, d) % 125]
         s[d, 3] = max((rnd_u64(seed ^ 0xABCDEF, env, d) >> 11), 1) / float(1 << 53) if setting == 3 else 1.0
     return s
+
+
+def obs_digest(obs):
+    """SHA-256 of the float64 values of an observation (-0.0 counted as 0.0) as 32 uint8: the reference records of
+    tests/golden/make_reference_records.py keep observations in this form, so that equal digests mean np.array_equal observations"""
+    a = np.ascontiguousarray(obs, dtype=np.float64) + 0.0
+    return np.frombuffer(hashlib.sha256(a.tobytes()).digest(), dtype=np.uint8)
+
+
+def obs_digests(obs_seq):
+    return np.stack([obs_digest(o) for o in obs_seq])
 
 
 # ---- non-default configurations (tests/golden/make_golden_cases.py records them from the reference; the GPU cases of

@@ -105,62 +105,47 @@ def test_facade_dataset_handling_continuous(fake, tmp_path):
     assert np.allclose([r[0] for r in rec], ratio[:5], rtol=0, atol=1e-12)
 
 
-# ---- the vector surface against the reference's OWN wrappers (build container only) ---------------------------------------------
+# ---- the vector surface against the reference's OWN wrappers ---------------------------------------------------------------------
 import ref_shim  # noqa: E402
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference not mounted")
 @pytest.mark.parametrize("setting", [1, 2])
-def test_vec_env_equals_reference_shmem_vecpytorch_monitor(fake, setting, tmp_path, monkeypatch):
+def test_vec_env_equals_reference_shmem_vecpytorch_monitor(fake, setting, monkeypatch):
     """VecPyTorch(ShmemVecEnv([Monitor(PackingDiscrete)] * N, context='fork')) of the unmodified reference (envs.py:75-116,159-182,
-    wrapper/shmem_vec_env.py, wrapper/monitor.py) next to PctVecEnv: observation tensors, reward shape / values, done array, info
-    dicts (terminal ones with Monitor's 'episode' entry, the auto-reset observation) over 70 vector steps."""
-    from harness import make_stream, policy_pick
+    wrapper/shmem_vec_env.py, wrapper/monitor.py), recorded by tests/golden/make_reference_records.py, next to PctVecEnv: observation
+    tensors, reward shape / values, done array, info dicts (terminal ones with Monitor's 'episode' entry, the auto-reset observation) over
+    70 vector steps."""
+    from harness import make_stream, obs_digests, policy_pick
     monkeypatch.setattr(importlib.import_module("pct_b200.vec_env"), "PctBatch", FakeBatch)
     import pct_b200
-    D, _ = ref_shim.load_reference()
-    renvs = importlib.import_module("envs")
-    ShmemVecEnv = importlib.import_module("wrapper.shmem_vec_env").ShmemVecEnv
-    Monitor = importlib.import_module("wrapper.monitor").Monitor
+    g = np.load(os.path.join(G, "vecenv_s%d.npz" % setting))
     n, seed = 5, 50 + setting
     streams = np.stack([make_stream(seed, e, 300, setting) for e in range(n)])
-
-    def thunk(rank):
-        def _t():
-            env = D.PackingDiscrete(setting=setting, container_size=[10, 10, 10], item_set=ITEM_SET, internal_node_holder=80, leaf_node_holder=50,
-                                    shuffle=False, LNES="EMS")
-            env.box_creator = ref_shim.make_stream_creator(D, [tuple(int(v) for v in r[:3]) for r in streams[rank]])
-            env.test = True
-            return Monitor(env, os.path.join(str(tmp_path), str(rank)), allow_early_resets=True)
-        return _t
-
-    probe = D.PackingDiscrete(setting=setting, container_size=[10, 10, 10], item_set=ITEM_SET)
-    ref = renvs.VecPyTorch(ShmemVecEnv([thunk(r) for r in range(n)], [probe.observation_space, probe.action_space], context="fork"), "cpu")
     ours = pct_b200.PctVecEnv(n, setting, item_set=ITEM_SET, item_stream=streams)
     try:
-        o_ref, o = ref.reset(), ours.reset()
-        assert o_ref.dtype == o.dtype == torch.float32 and tuple(o.shape) == tuple(o_ref.shape) == (n, 1179)
+        o = ours.reset()
+        assert o.dtype == torch.float32 and tuple(o.shape) == (n, 1179)  # the reference's VecPyTorch observations: float32, (n, 1179)
         dones = 0
         for t in range(70):
-            assert torch.equal(o_ref, o), "observations before step %d" % t
-            rows = np.stack([policy_pick(o_ref[e].numpy().astype(np.float64), 80, 50, seed, e, t)[1] for e in range(n)]).astype(np.float32)
-            o_ref, r_ref, d_ref, i_ref = ref.step(rows)  # float32 numpy leaf rows, as train_tools.py:66-67 passes them
-            o, r, d, i = ours.step(rows)
+            assert np.array_equal(g["obs"][t], obs_digests(o.cpu().numpy())), "observations before step %d" % t
+            rows = np.stack([policy_pick(o[e].cpu().numpy().astype(np.float64), 80, 50, seed, e, t)[1] for e in range(n)]).astype(np.float32)
+            o, r, d, i = ours.step(rows)  # float32 numpy leaf rows, as train_tools.py:66-67 passes them
+            r_ref, d_ref = torch.from_numpy(g["reward"][t]), g["done"][t]
             assert tuple(r.shape) == tuple(r_ref.shape) == (n, 1) and r.dtype == r_ref.dtype and torch.equal(r, r_ref)
             assert d.dtype == d_ref.dtype == np.bool_ and np.array_equal(d, d_ref)
             for e in range(n):
-                assert i[e]["counter"] == i_ref[e]["counter"]
+                keys_ref = set(str(g["info_keys"][t, e]).split(","))
+                assert i[e]["counter"] == g["counter"][t, e]
                 if d_ref[e]:
                     dones += 1
-                    assert set(i_ref[e]) == set(i[e]) == {"counter", "ratio", "reward", "episode"}
-                    assert abs(i[e]["ratio"] - i_ref[e]["ratio"]) < 1e-6 and abs(i[e]["reward"] - i_ref[e]["reward"]) < 1e-5
-                    assert i[e]["episode"]["l"] == i_ref[e]["episode"]["l"] and abs(i[e]["episode"]["r"] - i_ref[e]["episode"]["r"]) < 1e-4
+                    assert keys_ref == set(i[e]) == {"counter", "ratio", "reward", "episode"}
+                    assert abs(i[e]["ratio"] - g["ratio"][t, e]) < 1e-6 and abs(i[e]["reward"] - g["info_reward"][t, e]) < 1e-5
+                    assert i[e]["episode"]["l"] == g["ep_l"][t, e] and abs(i[e]["episode"]["r"] - g["ep_r"][t, e]) < 1e-4
                 else:
-                    assert set(i[e]) == set(i_ref[e]) == {"counter"}
+                    assert set(i[e]) == keys_ref == {"counter"}
+        assert np.array_equal(g["obs"][70], obs_digests(o.cpu().numpy()))
         assert dones >= 8
     finally:
-        ref.close()
         ours.close()
 
 
@@ -231,17 +216,19 @@ def test_unmodified_heuristic_functions_run_on_the_continuous_facade(fake, name,
     assert env.log[:3] == packed[:3]
 
 
-@pytest.mark.reference
-@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference not mounted")
 @pytest.mark.parametrize("argv,continuous", [(["--setting", "1", "--num-processes", "6", "--seed", "9"], False),
                                               (["--setting", "2", "--continuous", "--sample-from-distribution", "--num-processes", "4"], True)])
 def test_make_vec_envs_takes_the_reference_args(fake, argv, continuous, monkeypatch):
-    """envs.make_vec_envs(args, log_dir, allow_early_resets) (envs.py:75-116) with the namespace tools.get_args() builds"""
+    """envs.make_vec_envs(args, log_dir, allow_early_resets) (envs.py:75-116) with the namespace tools.get_args() builds from `argv`
+    (recorded from the reference by tests/golden/make_reference_records.py)"""
+    import argparse
+    import json
     import pct_b200
-    from pct_oracle import OracleBatch
-    compat = importlib.import_module("pct_b200.compat")
     monkeypatch.setattr(importlib.import_module("pct_b200.vec_env"), "PctBatch", FakeBatch)
-    args = compat.reference_args(ref_shim.REFERENCE_ROOT, argv)
+    with open(os.path.join(G, "reference_args.json")) as f:
+        rec = json.load(f)["continuous" if continuous else "discrete"]
+    assert rec["argv"] == argv
+    args = argparse.Namespace(**rec["args"])
     if continuous:
         args.container_size = [1, 1, 1]  # givenData.py:5 (the commented alternative)
         args.sample_left_bound, args.sample_right_bound = 0.1, 0.5

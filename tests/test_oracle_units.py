@@ -1,6 +1,7 @@
 """CPU: the oracle's building blocks against CPython / numpy themselves (third-party arithmetic the reference leans on:
-set iteration order, tuple and float hashes, lstsq) and against the reference's convex_hull.py when it is mounted."""
+set iteration order, tuple and float hashes, lstsq) and against records of the reference's convex_hull.py."""
 import ctypes as C
+import os
 import random
 
 import numpy as np
@@ -74,23 +75,20 @@ def test_lstsq_rank_deficient_minimum_norm():
     assert np.allclose(x, want, rtol=1e-6, atol=1e-9)
 
 
-@pytest.mark.reference
 def test_hull_and_pip_match_reference_module():
-    import ref_shim
-    if not ref_shim.reference_available():
-        pytest.skip("reference not mounted")
-    D, _ = ref_shim.load_reference()
-    from pct_envs.PctDiscrete0.convex_hull import ConvexHull, point_in_polygen
-    from pct_envs.PctDiscrete0.space import Space
-    sp = Space(10, 10, 10, 1, 80)
+    """oracle hull / point-in-polygon against the reference's ConvexHull + Space.scale_down and point_in_polygen on the same random draws
+    (records of tests/golden/make_reference_records.py)"""
+    g = np.load(os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden", "hull_pip.npz"))
+    off = np.concatenate([[0], np.cumsum(g["hull_len"])])
     rng = np.random.RandomState(3)
+    n_pip = 0
     for trial in range(600):
         k = rng.choice([1, 1, 2, 2, 3, 4, 6])
         pts = []
         for _ in range(k):
             x1, y1 = rng.randint(0, 8, 2); x2, y2 = x1 + rng.randint(1, 4), y1 + rng.randint(1, 4)
             pts += [[x1, y1], [x1, y2], [x2, y1], [x2, y2]]
-        want = np.array(sp.scale_down(ConvexHull([list(p) for p in pts])))
+        want = g["hull_flat"][off[trial]:off[trial + 1]]
         p = np.array(pts, dtype=np.float64)
         out = np.zeros((2 * len(pts), 2))
         m = L.pcto_hull_shrunk(p.ctypes.data_as(C.POINTER(C.c_double)), len(pts), out.ctypes.data_as(C.POINTER(C.c_double)))
@@ -98,7 +96,9 @@ def test_hull_and_pip_match_reference_module():
         for _ in range(6):
             q = np.array([rng.randint(0, 20) / 2.0, rng.randint(0, 20) / 2.0]) if rng.rand() < 0.5 else rng.uniform(0, 10, 2)
             got = L.pcto_pip(q[0], q[1], np.ascontiguousarray(want).ctypes.data_as(C.POINTER(C.c_double)), m)
-            assert bool(got) == bool(point_in_polygen(q, want.tolist()))
+            assert bool(got) == bool(g["pip"][n_pip])
+            n_pip += 1
+    assert n_pip == len(g["pip"])
 
 
 def test_around6_commutes_with_min():

@@ -1,24 +1,25 @@
-"""CPU, build container only: the reference's OWN policy network and evaluation loop on the drop-in env surface.
+"""CPU: the reference's OWN policy network and evaluation loop on the drop-in env surface.
 
-`model.DRL_GAT` (attention_model.AttentionModel + graph encoder, loaded unmodified through oracle/ref_shim.load_policy_module) is
-driven with the calls of evaluation_tools.evaluate (:9-24: tools.get_leaf_nodes_with_factor on the observation, PCT_policy(all_nodes,
-True, normFactor), `leaf_nodes[batchX, idx]`, `env.step(row[0:6])`, `env.packed`) once on the reference env and once on an env with the
-facade's call surface.  There is no GPU in this container, so the CPU oracle stands in for the CUDA path here — the GPU parity tests
-assert the two produce bit-identical observations, which is all the policy ever sees.  Equal trajectories = the observation layout,
-the mask column, the 6-float action rows and `packed` are what the unmodified consumers expect.  Skipped without /root/reference."""
+`model.DRL_GAT` (attention_model.AttentionModel + graph encoder) driven with the calls of evaluation_tools.evaluate (:9-24:
+tools.get_leaf_nodes_with_factor on the observation, PCT_policy(all_nodes, True, normFactor), `leaf_nodes[batchX, idx]`, `env.step(row[0:6])`,
+`env.packed`) on the reference env is recorded by tests/golden/make_reference_records.py: every observation, the leaf index the network
+chose and each episode's (ratio, counter, packed).  The same choices are replayed on an env with the facade's call surface.  The CPU
+oracle stands in for the CUDA path here — the GPU parity tests assert the two produce bit-identical observations, which is all the policy
+ever sees, and equal observations mean the network would choose the same leaves.  Equal trajectories = the observation layout, the mask
+column, the 6-float action rows and `packed` are what the unmodified consumers expect.  test_compat_runs_the_unmodified_evaluate runs the
+reference's own code and is skipped without the reference checkout."""
 import os
 import sys
-import types
 
 import numpy as np
 import pytest
 
 import ref_shim
-from harness import ITEM_SET, make_stream
+from harness import make_stream, obs_digests
 from pct_oracle import OracleDiscrete
 
-sys.path.insert(0, os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden"))
-pytestmark = [pytest.mark.reference, pytest.mark.skipif(not ref_shim.reference_available(), reason="reference not mounted")]
+G = os.path.join(os.path.dirname(os.path.abspath(__file__)), "golden")
+sys.path.insert(0, G)
 torch = pytest.importorskip("torch")
 
 
@@ -31,49 +32,36 @@ def _one_torch_thread():
     torch.set_num_threads(n)
 
 
-def _policy(setting):
-    model, tools = ref_shim.load_policy_module()
-    args = types.SimpleNamespace(embedding_size=64, hidden_size=128, gat_layer_num=1, internal_node_holder=80,
-                                 internal_node_length=7 if setting == 3 else 6, leaf_node_holder=50)  # tools.py:148-190 defaults
-    torch.manual_seed(1234 + setting)
-    return model.DRL_GAT(args).eval(), tools
-
-
-def _episodes(env, policy, tools, n_episodes, factor):
-    """the body of evaluation_tools.evaluate (:9-41) for one env"""
+def _replay(env, leaf_idx, n_episodes):
+    """the body of evaluation_tools.evaluate (:9-41) for one env, with the leaf indices the reference's network chose"""
     out, traj = [], []
     obs = env.reset()
-    while len(out) < n_episodes:
-        obs_t = torch.FloatTensor(obs).unsqueeze(dim=0)
-        all_nodes, leaf_nodes = tools.get_leaf_nodes_with_factor(obs_t, 1, 80, 50)
-        with torch.no_grad():
-            _, idx, _, _ = policy(all_nodes, True, normFactor=factor)
-        row = leaf_nodes[torch.arange(1), idx.squeeze()].cpu().numpy()[0][0:6]
+    for idx in leaf_idx:
+        row = np.asarray(obs, dtype=np.float32).reshape(-1, 9)[80 + idx][0:6]  # torch.FloatTensor(obs) -> leaf_nodes[0, idx][0:6]
         items = env.packed
         traj.append(np.asarray(obs).copy())
         obs, reward, done, infos = env.step(row)
         if done:
             out.append((infos["ratio"], infos["counter"], [list(map(float, p)) for p in items]))
             obs = env.reset()
+    assert len(out) == n_episodes
     return out, np.array(traj)
 
 
 @pytest.mark.parametrize("setting", [1, 2, 3])
 def test_reference_policy_and_eval_loop_on_the_drop_in_surface(setting):
-    D, _ = ref_shim.load_reference()
-    policy, tools = _policy(setting)
+    g = np.load(os.path.join(G, "policy_eval_s%d.npz" % setting))
+    off = np.concatenate([[0], np.cumsum(g["packed_len"])])
+    a = [(float(g["ratio"][e]), int(g["counter"][e]), g["packed_flat"][off[e]:off[e + 1]].tolist()) for e in range(len(g["ratio"]))]
     stream = make_stream(600 + setting, 0, 500, setting)
-    ref = D.PackingDiscrete(setting=setting, container_size=[10, 10, 10], item_set=ITEM_SET, internal_node_holder=80, leaf_node_holder=50,
-                            shuffle=False, LNES="EMS")
-    ref.box_creator = ref_shim.make_stream_creator(D, [tuple(r) if setting == 3 else tuple(int(v) for v in r[:3]) for r in stream])
-    ref.test = True
-    a, ta = _episodes(ref, policy, tools, 4, 0.1)
-    b, tb = _episodes(OracleDiscrete(setting, stream=stream), policy, tools, 4, 0.1)
-    assert np.array_equal(ta, tb)
+    b, tb = _replay(OracleDiscrete(setting, stream=stream), g["leaf_idx"], 4)
+    assert np.array_equal(g["traj"], obs_digests(tb))
     assert [(x[0], x[1]) for x in a] == [(x[0], x[1]) for x in b] and [x[2] for x in a] == [x[2] for x in b]
     assert min(x[1] for x in a) >= 5  # the argmax policy of a random-init network still packs several items per episode
 
 
+@pytest.mark.reference
+@pytest.mark.skipif(not ref_shim.reference_available(), reason="reference not mounted")
 def test_compat_runs_the_unmodified_evaluate(tmp_path):
     """pct_b200.compat: evaluation.py:10-56 around the UNMODIFIED evaluation_tools.evaluate (policy forward, env.step(row[0:6]), env.packed,
     trajs.npy, result.txt) — once on the reference env, once on an env with the facade's surface (oracle-backed here) — same files."""
