@@ -191,6 +191,36 @@ int pct_query_placement(pct_handle h, int32_t env, const int32_t dims[3], int32_
 int pct_query_placement_f64(pct_handle h, int32_t env, const double dims[3], double lx, double ly, double density,
                             int32_t *feasible, double *rest_height);
 
+/* Saved env records: copy the state of environments, within a handle or between handles (search / lookahead from a branch point,
+ * checkpoint and resume, moving envs between shards or GPUs).  What a copy continues with is defined by item_env: every env draws its items
+ * from the sequence of ONE global env id — its own (cfg.env_id_base + e) until a record is loaded into it, then the source's, kept across
+ * resets.  So "load the source's record into env d, then apply the same actions" gives exactly what the source gets, items drawn after the
+ * load included.  The random policy and PCT_H_RANDOM keep drawing with the env's own id: they are policy randomness, not env state.
+ *
+ * A record is an opaque, fixed-size (pct_env_record_bytes), 16-byte-aligned device slot per env.  It holds the env's live state (boxes, EMS,
+ * leaves of the last observation, item source position, episode sums, flags, load edges, the LSAH footprint) and a header with a 64-bit
+ * fingerprint of the configuration: domain, setting, container, holders, lnes, shuffle, seed, item mode, size_minimum, sample bounds,
+ * trajectory length, no_auto_reset, the item set contents, the stream length and the alias mode.  It leaves out env_id_base and obs_dtype,
+ * so records move between shards, GPUs and observation dtypes.  In stream mode the record also carries the content hash of the stream row it
+ * draws from.
+ *
+ * Both calls only enqueue stream-ordered work on `stream`: no host synchronisation, no allocation (CUDA-graph capturable). */
+int64_t pct_env_record_bytes(pct_handle h);
+/* d_records[i] = record of env d_env_ids[i], i < n.  Ids may repeat (saving repeat_interleave(src, K) gives K copies of each source);
+ * d_env_ids == NULL: n == n_envs, record i = env i.  An id outside [0, n_envs) writes a record with an invalid header (it loads nowhere). */
+int pct_save_envs(pct_handle h, const int32_t *d_env_ids, int32_t n, void *d_records, void *stream);
+/* env d_env_ids[i] = the state in d_records[i], i < n (d_env_ids == NULL: n == n_envs, env i).  Each record is checked against the handle
+ * before anything is written; d_status (n int32, may be NULL) receives per record
+ *   0  loaded
+ *   1  not a record of this configuration (header, version, domain or fingerprint differ; stream mode: the stream row differs)
+ *   2  stream mode: the item row the record draws from (item_env - cfg.env_id_base) is not one of this handle's rows
+ *   3  destination env id outside [0, n_envs)
+ * and a rejected record leaves its destination untouched.  Destination ids must be distinct within one call (duplicates: undefined).
+ * d_obs (n_envs x obs_len of cfg.obs_dtype, may be NULL) receives the full observation rows of the loaded envs (their source's last
+ * observation, terminal ones of a no_auto_reset handle included); whatever buffer the next pct_step gets, it rewrites every row of the
+ * loaded envs, so the delta-row contract of pct_step holds.  Needs a handle that has been reset (else PCT_ERR_STATE). */
+int pct_load_envs(pct_handle h, const int32_t *d_env_ids, int32_t n, const void *d_records, void *d_obs, int32_t *d_status, void *stream);
+
 /* introspection */
 int pct_get_state(pct_handle h, int32_t env, pct_state_dump *out);
 int32_t pct_obs_len(pct_handle h);       /* (NB + NL + 1) * 9 */

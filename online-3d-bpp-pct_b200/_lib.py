@@ -41,7 +41,8 @@ class StateDump(C.Structure):
 EXPORTS = ["pct_create", "pct_destroy", "pct_last_error", "pct_set_item_set", "pct_set_item_stream", "pct_set_trajectory_length", "pct_reset", "pct_step",
            "pct_step_host", "pct_reset_host", "pct_policy_random", "pct_policy_random_dev", "pct_get_state", "pct_obs_len", "pct_num_envs",
            "pct_state_bytes_per_env", "pct_kernel_launches", "pct_version", "pct_profile_enable", "pct_profile_read", "pct_heuristic_actions",
-           "pct_heuristic_actions_f64", "pct_query_placement", "pct_query_placement_f64"]
+           "pct_heuristic_actions_f64", "pct_query_placement", "pct_query_placement_f64", "pct_env_record_bytes", "pct_save_envs", "pct_load_envs"]
+RECORD_STATUS = {1: "not a record of this configuration", 2: "item-stream row not in this handle", 3: "env id out of range"}  # pct_load_envs
 
 
 def build(verbose=False):
@@ -91,5 +92,9 @@ def lib():
     L.pct_query_placement.argtypes = [vp, i32, C.POINTER(i32), i32, i32, C.c_double, C.POINTER(i32), C.POINTER(i32), C.POINTER(i32)]
     L.pct_query_placement_f64.argtypes = [vp, i32, C.POINTER(C.c_double), C.c_double, C.c_double, C.c_double, C.POINTER(i32),
                                           C.POINTER(C.c_double)]
+    L.pct_env_record_bytes.argtypes = [vp]
+    L.pct_env_record_bytes.restype = i64
+    L.pct_save_envs.argtypes = [vp, vp, i32, vp, vp]
+    L.pct_load_envs.argtypes = [vp, vp, i32, vp, vp, vp, vp]
     _lib = L
     return L

@@ -16,6 +16,47 @@ class PctError(RuntimeError):
     pass
 
 
+def record_arguments(records, env_ids, n_envs, record_bytes, device):
+    """Checks and normalises the arguments of PctBatch.load_envs: -> (records, env ids or None, n).  records: (n, record_bytes) uint8, moved to
+    `device` when they live elsewhere; env_ids: None (n == n_envs, record i -> env i) or n distinct ids in [0, n_envs) as a contiguous int32
+    tensor on `device`.  Raises PctError."""
+    if not isinstance(records, torch.Tensor):
+        raise PctError("records must be a tensor (the output of save_envs)")
+    if records.dtype != torch.uint8 or records.dim() != 2 or records.shape[1] != record_bytes:
+        raise PctError("records must be a (n, %d) uint8 tensor, got %s %s" % (record_bytes, tuple(records.shape), records.dtype))
+    if records.device != device:
+        records = records.to(device)
+    records = records.contiguous()
+    n = int(records.shape[0])
+    ids = env_id_tensor(env_ids, n_envs, device)
+    if ids is None:
+        if n != n_envs:
+            raise PctError("records for all %d envs expected without env_ids, got %d" % (n_envs, n))
+    else:
+        if ids.numel() != n:
+            raise PctError("%d records for %d env ids" % (n, ids.numel()))
+        if n and (int(ids.min()) < 0 or int(ids.max()) >= n_envs):
+            raise PctError("env ids must lie in [0, %d)" % n_envs)
+        if torch.unique(ids).numel() != n:
+            raise PctError("duplicate destination env ids in one load")
+    return records, ids, n
+
+
+def env_id_tensor(env_ids, n_envs, device):
+    """None, or env ids (tensor / sequence of integers) as a contiguous 1-D int32 tensor on `device`"""
+    if env_ids is None:
+        return None
+    if isinstance(env_ids, torch.Tensor):
+        if env_ids.dtype.is_floating_point or env_ids.dtype == torch.bool:
+            raise PctError("env ids must be integers, got %s" % env_ids.dtype)
+        ids = env_ids
+    else:
+        ids = torch.as_tensor(np.asarray(env_ids, dtype=np.int64))
+    if ids.dim() != 1:
+        raise PctError("env ids must be a 1-D sequence")
+    return ids.to(device=device, dtype=torch.int32).contiguous()
+
+
 class PctBatch(object):
     def __init__(self, n_envs, setting, container_size=(10, 10, 10), item_set=None, internal_node_holder=80,
                  leaf_node_holder=50, continuous=False, obs_dtype=torch.float32, seed=0, env_id_base=0, device=0,
@@ -147,6 +188,64 @@ class PctBatch(object):
         self._check(self.L.pct_policy_random_dev(self.h, C.c_void_p(idx.data_ptr()), int(seed) & ((1 << 64) - 1), C.c_void_p(t_dev.data_ptr()),
                                                  self._stream()), "pct_policy_random_dev")
         return idx
+
+    # -- saved env records (include/pct_b200.h, pct_save_envs / pct_load_envs) ----------------------------------------
+    @property
+    def record_bytes(self):
+        """size of one saved env record (fixed per domain)"""
+        return int(self.L.pct_env_record_bytes(self.h))
+
+    def save_envs(self, env_ids=None, out=None):
+        """The state of the envs `env_ids` (repeats allowed: repeat_interleave(src, K) gives K copies of each source; None = every env in order)
+        as a (n, record_bytes) uint8 CUDA tensor (or into `out`).  The records are opaque; load_envs puts them into this or any handle with the
+        same configuration (another env_id_base, GPU or observation dtype included).  Enqueued on the current stream, no synchronisation."""
+        ids = env_id_tensor(env_ids, self.n_envs, self.device)
+        n = self.n_envs if ids is None else int(ids.numel())
+        rb = self.record_bytes
+        if out is None:
+            out = torch.empty((n, rb), dtype=torch.uint8, device=self.device)
+        if out.dtype != torch.uint8 or tuple(out.shape) != (n, rb) or not out.is_contiguous() or out.device != self.device:
+            raise PctError("out must be a contiguous (%d, %d) uint8 tensor on %s" % (n, rb, self.device))
+        self._check(self.L.pct_save_envs(self.h, C.c_void_p(ids.data_ptr()) if ids is not None else None, n, C.c_void_p(out.data_ptr()),
+                                         self._stream()), "pct_save_envs")
+        return out
+
+    def load_envs(self, records, env_ids=None, obs=None, check=True, status=None):
+        """Env env_ids[i] takes the state saved in records[i] (None: record i -> env i) and continues exactly like its source, items drawn after the
+        load included.  obs: an (n_envs, obs_len) tensor of the handle's observation dtype that receives the loaded envs' observation rows.
+        check=True synchronises and raises PctError when a record does not belong to this configuration (or, in item-stream mode, draws from a
+        stream row this handle does not hold), and rejects duplicate destination ids.  check=False does not synchronise (CUDA-graph capture):
+        pass `status` (n int32 on the device) to get the per-record codes (0 loaded, 1 other configuration, 2 stream row not here, 3 bad env
+        id); a rejected record leaves its env untouched.  Returns the status tensor (None with check=False and no `status`)."""
+        if check:
+            records, ids, n = record_arguments(records, env_ids, self.n_envs, self.record_bytes, self.device)
+        else:  # no host synchronisation: shape checks only
+            if records.device != self.device:
+                records = records.to(self.device)
+            records = records.contiguous()
+            n = int(records.shape[0])
+            if records.dtype != torch.uint8 or records.dim() != 2 or records.shape[1] != self.record_bytes:
+                raise PctError("records must be a (n, %d) uint8 tensor" % self.record_bytes)
+            ids = env_id_tensor(env_ids, self.n_envs, self.device)
+            if ids is not None and ids.numel() != n:
+                raise PctError("%d records for %d env ids" % (n, ids.numel()))
+        if obs is not None and (obs.dtype != self.obs_dtype or tuple(obs.shape) != (self.n_envs, self.obs_len) or not obs.is_contiguous()
+                                or obs.device != self.device):
+            raise PctError("obs must be a contiguous (%d, %d) %s tensor on %s" % (self.n_envs, self.obs_len, self.obs_dtype, self.device))
+        if status is None and check:
+            status = torch.empty((n,), dtype=torch.int32, device=self.device)
+        if status is not None and (status.dtype != torch.int32 or status.numel() < n or not status.is_contiguous() or status.device != self.device):
+            raise PctError("status must be a contiguous int32 tensor of >= %d elements on %s" % (n, self.device))
+        self._check(self.L.pct_load_envs(self.h, C.c_void_p(ids.data_ptr()) if ids is not None else None, n, C.c_void_p(records.data_ptr()),
+                                         C.c_void_p(obs.data_ptr()) if obs is not None else None,
+                                         C.c_void_p(status.data_ptr()) if status is not None else None, self._stream()), "pct_load_envs")
+        if check:
+            st = status[:n].cpu().numpy()
+            if st.any():
+                bad = np.nonzero(st)[0]
+                raise PctError("pct_load_envs rejected %d of %d record(s) (first: record %d, status %d = %s); rejected records left their envs untouched"
+                               % (len(bad), n, int(bad[0]), int(st[bad[0]]), _lib.RECORD_STATUS.get(int(st[bad[0]]), "?")))
+        return status
 
     # -- heuristic baselines (heuristic.py) ------------------------------------------------------------------
     def heuristic_actions(self, name, seed=0, t=0, out=None):

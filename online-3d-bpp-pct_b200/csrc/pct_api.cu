@@ -6,6 +6,7 @@
 #include <string>
 #include <vector>
 
+#include "pct_common.cuh"  // splitmix64
 #include "pct_kernels.h"
 #include "pct_handle.h"
 
@@ -34,7 +35,33 @@ int continuous_get_state(pct_env_batch *h, int env, pct_state_dump *out);
 int64_t continuous_state_bytes();
 int continuous_heuristic(pct_env_batch *h, int code, double *rows, double *hstate, cudaStream_t st);
 int continuous_query(pct_env_batch *h, int env, const double q[5], double density, double *d_out, cudaStream_t st);
+int64_t continuous_record_bytes();
+int continuous_records(pct_env_batch *h, const RecArgs &s, int load, void *obs, cudaStream_t st);
 }  // namespace pct
+
+// 64-bit FNV-1a over byte ranges, finished with splitmix64 (host side: configuration fingerprint, item set / stream row hashes)
+static uint64_t fnv1a(uint64_t hash, const void *data, size_t n) {
+    const unsigned char *b = (const unsigned char *)data;
+    for (size_t i = 0; i < n; i++) { hash ^= b[i]; hash *= 0x100000001B3ull; }
+    return hash;
+}
+constexpr uint64_t FNV_SEED = 0xCBF29CE484222325ull;
+
+// Everything that gives a saved env record its meaning: a record loads only into a handle with the same fingerprint.  Leaves out
+// env_id_base (records move between shards: item_env keeps the item sequence) and obs_dtype (the record holds no observation).
+static uint64_t config_fingerprint(pct_handle h) {
+    const pct_config &c = h->cfg;
+    uint64_t f = FNV_SEED;
+    auto mix = [&](const auto &v) { f = fnv1a(f, &v, sizeof v); };
+    mix(c.domain); mix(c.setting); mix(c.container_size); mix(c.internal_node_holder); mix(c.leaf_node_holder); mix(c.lnes); mix(c.shuffle);
+    mix(c.seed); mix(h->item_mode); mix(c.size_minimum); mix(c.sample_from_distribution); mix(c.sample_left_bound); mix(c.sample_right_bound);
+    mix(h->traj_len); mix(c.no_auto_reset);
+    mix(h->n_items); mix(h->item_set_hash);  // item set contents
+    mix(h->stream_len);                      // item stream: its rows are checked one by one (RecHdr::row_hash)
+    const int32_t alias = h->alias_mode ? 1 : 0;  // PCT_B200_ALIAS=0 handles do not maintain DEnvAux::box_st
+    mix(alias);
+    return splitmix64(f);
+}
 
 extern "C" {
 
@@ -104,6 +131,10 @@ int pct_create(const pct_config *cfg, int32_t n_envs, int32_t device, pct_handle
     if (const char *wv = getenv("PCT_B200_WALK_BLOCKS")) { h->walk_blocks = atoi(wv); if (h->walk_blocks < 1) h->walk_blocks = 1; if (h->walk_blocks > 8) h->walk_blocks = 8; }
     if (const char *wv = getenv("PCT_B200_WALK_LANES")) { h->walk_lanes = atoi(wv); if (h->walk_lanes < 1) h->walk_lanes = 1; if (h->walk_lanes > 32) h->walk_lanes = 32; }
     if (cfg->setting == 2) h->alias_mode = false;  // no stability check, no load entries
+    // LSAH footprint state: per-env state that saved records carry, allocated here so that a load never allocates
+    const size_t hs_bytes = (cfg->domain == PCT_CONTINUOUS ? sizeof(double) : sizeof(int32_t)) * 4 * (size_t)n_envs;
+    if (e == cudaSuccess) e = cudaMalloc(cfg->domain == PCT_CONTINUOUS ? (void **)&h->d_hstate_c : (void **)&h->d_hstate, hs_bytes);
+    if (e == cudaSuccess) e = cudaMemset(cfg->domain == PCT_CONTINUOUS ? (void *)h->d_hstate_c : (void *)h->d_hstate, 0, hs_bytes);
     if ((h->obs_delta || h->alias_mode) && e == cudaSuccess) {
         e = cudaMalloc(&h->d_aux, sizeof(DEnvAux) * (size_t)n_envs);
         if (e == cudaSuccess) e = cudaMemset(h->d_aux, 0, sizeof(DEnvAux) * (size_t)n_envs);
@@ -126,6 +157,12 @@ int pct_create(const pct_config *cfg, int32_t n_envs, int32_t device, pct_handle
             e = cudaMalloc(&h->d_hot, sizeof(DEnvHot) * (size_t)n_envs);
             if (e == cudaSuccess) e = cudaMalloc(&h->d_cold, sizeof(DEnvCold) * (size_t)n_envs);
             if (e == cudaSuccess) e = cudaMemset(h->d_hot, 0, sizeof(DEnvHot) * (size_t)n_envs);
+            if (e == cudaSuccess) {  // item_env = the env's own global id (DHdr::item_env)
+                std::vector<int64_t> id((size_t)n_envs);
+                for (int i = 0; i < n_envs; i++) id[i] = cfg->env_id_base + i;
+                e = cudaMemcpy2D((char *)h->d_hot + offsetof(DEnvHot, h) + offsetof(DHdr, item_env), sizeof(DEnvHot), id.data(), sizeof(int64_t),
+                                 sizeof(int64_t), (size_t)n_envs, cudaMemcpyHostToDevice);
+            }
             if (e == cudaSuccess) e = cudaMalloc(&h->d_ready, sizeof(int32_t) * 2 * (size_t)n_envs);
             if (e == cudaSuccess) e = cudaMemset(h->d_ready, 0, sizeof(int32_t) * 2 * (size_t)n_envs);
             if (e == cudaSuccess) e = cudaMemset(h->d_cold, 0, sizeof(DEnvCold) * (size_t)n_envs);
@@ -179,7 +216,7 @@ void pct_destroy(pct_handle h) {
     cudaFree(h->d_walkq); cudaFree(h->d_walk_ctr); cudaFree(h->d_contq); cudaFree(h->d_cont_ctr); cudaFree(h->d_piece_ready); cudaFree(h->d_walk_pend);
     cudaFree(h->d_hstate); cudaFree(h->d_hstate_c); cudaFree(h->d_query_c); cudaFree(h->d_query); cudaFree(h->d_aux);
     cudaFree(h->d_ready);
-    cudaFree(h->d_hot); cudaFree(h->d_cold); cudaFree(h->d_item_set); cudaFree(h->d_stream);
+    cudaFree(h->d_hot); cudaFree(h->d_cold); cudaFree(h->d_item_set); cudaFree(h->d_stream); cudaFree(h->d_row_hash);
     cudaFree(h->d_obs); cudaFree(h->d_act); cudaFree(h->d_idx); cudaFree(h->d_rew); cudaFree(h->d_done); cudaFree(h->d_info);
     for (cudaEvent_t ev : h->prof_ev) if (ev) cudaEventDestroy(ev);
     if (h->own_stream) cudaStreamDestroy(h->own_stream);
@@ -199,6 +236,7 @@ int pct_set_item_set(pct_handle h, const double *items_xyz, int32_t n_items) {
     CK(h, cudaMalloc(&h->d_item_set, sizeof(double) * 3 * (size_t)n_items));
     CK(h, cudaMemcpy(h->d_item_set, items_xyz, sizeof(double) * 3 * (size_t)n_items, cudaMemcpyHostToDevice));
     h->n_items = n_items;
+    h->item_set_hash = splitmix64(fnv1a(FNV_SEED, items_xyz, sizeof(double) * 3 * (size_t)n_items));
     return PCT_OK;
 }
 
@@ -210,6 +248,11 @@ int pct_set_item_stream(pct_handle h, const double *items_xyzd, int32_t len) {
     const size_t bytes = sizeof(double) * 4 * (size_t)len * (size_t)h->n_envs;
     CK(h, cudaMalloc(&h->d_stream, bytes));
     CK(h, cudaMemcpy(h->d_stream, items_xyzd, bytes, cudaMemcpyHostToDevice));
+    std::vector<uint64_t> rows((size_t)h->n_envs);
+    const size_t row_bytes = sizeof(double) * 4 * (size_t)len;
+    for (int i = 0; i < h->n_envs; i++) rows[i] = splitmix64(fnv1a(FNV_SEED, (const char *)items_xyzd + row_bytes * i, row_bytes));
+    if (!h->d_row_hash) CK(h, cudaMalloc(&h->d_row_hash, sizeof(uint64_t) * (size_t)h->n_envs));
+    CK(h, cudaMemcpy(h->d_row_hash, rows.data(), sizeof(uint64_t) * rows.size(), cudaMemcpyHostToDevice));
     h->stream_len = len;
     h->item_mode = PCT_ITEMS_STREAM;
     return PCT_OK;
@@ -486,10 +529,6 @@ int pct_heuristic_actions(pct_handle h, int32_t heuristic, float *d_rows, uint64
         h->err = "PCT_H_HM / PCT_H_MACS / PCT_H_RANDOM need container sides <= 32";
         return PCT_ERR_INVALID;
     }
-    if (!h->d_hstate) {
-        CK(h, cudaMalloc(&h->d_hstate, sizeof(int32_t) * 4 * (size_t)h->n_envs));
-        CK(h, cudaMemset(h->d_hstate, 0, sizeof(int32_t) * 4 * (size_t)h->n_envs));
-    }
     HParams hp{};
     hp.code = heuristic; hp.rows = d_rows; hp.hstate = h->d_hstate; hp.seed = seed; hp.t = t;
     CK(h, launch_heuristic_discrete(p, hp, (cudaStream_t)stream));
@@ -507,10 +546,6 @@ int pct_heuristic_actions_f64(pct_handle h, int32_t heuristic, double *d_rows, v
     if (!h->did_reset) { h->err = "pct_heuristic_actions_f64 before pct_reset"; return PCT_ERR_STATE; }
     if (heuristic == PCT_H_BR && !h->d_item_set) { h->err = "PCT_H_BR scores an EMS by the item types that fit: call pct_set_item_set"; return PCT_ERR_STATE; }
     CK(h, cudaSetDevice(h->device));
-    if (!h->d_hstate_c) {
-        CK(h, cudaMalloc(&h->d_hstate_c, sizeof(double) * 4 * (size_t)h->n_envs));
-        CK(h, cudaMemset(h->d_hstate_c, 0, sizeof(double) * 4 * (size_t)h->n_envs));
-    }
     int rc = continuous_heuristic(h, heuristic, d_rows, h->d_hstate_c, (cudaStream_t)stream);
     if (rc != PCT_OK) return rc;
     h->launches++;
@@ -583,6 +618,54 @@ int pct_get_state(pct_handle h, int32_t env, pct_state_dump *out) {
     for (int i = 0; i < hot.h.n_ems && i < 256 && i < E_MAX; i++)
         for (int t = 0; t < 6; t++) out->ems[i][t] = hot.ems[i][t];
     return PCT_OK;
+}
+
+int64_t pct_env_record_bytes(pct_handle h) {
+    if (!h) return 0;
+    return h->cfg.domain == PCT_CONTINUOUS ? continuous_record_bytes() : discrete_record_bytes();
+}
+
+// save (load == 0) / load (load == 1): argument checks, then one stream-ordered kernel; no host synchronisation, no allocation
+static int env_records(pct_handle h, const int32_t *d_env_ids, int32_t n, const void *d_records, void *d_obs, int32_t *d_status, void *stream,
+                       int load) {
+    const char *what = load ? "pct_load_envs" : "pct_save_envs";
+    if (!h) return PCT_ERR_INVALID;
+    if (n < 0 || (n > 0 && !d_records) || (!d_env_ids && n != h->n_envs && n != 0)) {
+        h->err = std::string(what) + ": bad arguments (d_env_ids == NULL means all n_envs envs in order)";
+        return PCT_ERR_INVALID;
+    }
+    if (((uintptr_t)d_records & 15) != 0) { h->err = std::string(what) + ": records must be 16-byte aligned"; return PCT_ERR_INVALID; }
+    if (load && !h->did_reset) { h->err = "pct_load_envs before pct_reset"; return PCT_ERR_STATE; }
+    CK(h, cudaSetDevice(h->device));
+    RecArgs s{};
+    s.ids = d_env_ids; s.n = n; s.rec = (unsigned char *)const_cast<void *>(d_records); s.rec_bytes = pct_env_record_bytes(h);
+    s.fingerprint = config_fingerprint(h);
+    s.row_hash = h->item_mode == PCT_ITEMS_STREAM ? h->d_row_hash : nullptr;
+    s.alias = h->alias_mode && h->d_aux && h->cfg.setting != 2;
+    s.status = d_status;
+    const cudaStream_t st = (cudaStream_t)stream;
+    if (h->cfg.domain == PCT_CONTINUOUS) {
+        s.hstate = h->d_hstate_c;
+        const int rc = continuous_records(h, s, load, load ? d_obs : nullptr, st);
+        if (rc == PCT_OK && n > 0) h->launches++;
+        return rc;
+    }
+    s.hstate = h->d_hstate;
+    DParams p = state_params(h);
+    p.aux = h->d_aux;
+    p.obs = load ? d_obs : nullptr;
+    p.obs_f64 = h->cfg.obs_dtype == PCT_F64;
+    CK(h, launch_records_discrete(p, s, load, st));
+    if (n > 0) h->launches++;
+    return PCT_OK;
+}
+
+int pct_save_envs(pct_handle h, const int32_t *d_env_ids, int32_t n, void *d_records, void *stream) {
+    return env_records(h, d_env_ids, n, d_records, nullptr, nullptr, stream, 0);
+}
+
+int pct_load_envs(pct_handle h, const int32_t *d_env_ids, int32_t n, const void *d_records, void *d_obs, int32_t *d_status, void *stream) {
+    return env_records(h, d_env_ids, n, d_records, d_obs, d_status, stream, 1);
 }
 
 int32_t pct_obs_len(pct_handle h) { return h ? h->obs_len : 0; }

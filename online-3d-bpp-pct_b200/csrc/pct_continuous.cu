@@ -16,6 +16,7 @@
 #include "pct_handle.h"
 #include "pct_geom_continuous.cuh"
 #include "pct_walkq.cuh"
+#include "pct_records.cuh"
 
 namespace pct {
 
@@ -31,6 +32,7 @@ struct CHdr {
     double next_den;
     double vol_sum;
     int32_t ep_len, n_cand, n_edge, n_poly;
+    int64_t item_env;   // global env id whose item sequence this env follows (its own id unless a saved record was loaded into it)
 };
 struct alignas(16) CEnv {
     CHdr h;
@@ -40,6 +42,7 @@ struct alignas(16) CEnv {
     double ems_tmp[CE_TMP][6];
     uint16_t e_off[NB_MAX + 2], poly_off[NB_MAX + 2];
     uint8_t e_lower[EDGE_MAX + 1], e_next[EDGE_MAX + 1], first_in[NB_MAX], last_in[NB_MAX];
+    uint8_t pad_topo_[8];         // keeps e_st / poly / leaf 16-byte aligned (saved records copy them in 16-byte units)
     Stack4 e_st[EDGE_MAX + 1];
     double poly[POLY_MAX][2];
     double leaf[NL_MAX][6];
@@ -125,7 +128,7 @@ __device__ __noinline__ uint64_t cand_hash_c(const double t[6]) {
 }
 
 __device__ __noinline__ void draw_item_c(const CParams &p, int e, CHdr &h) {
-    const uint64_t gid = (uint64_t)(p.env_id_base + e), d = (uint64_t)h.draw_pos;
+    const uint64_t gid = (uint64_t)h.item_env, d = (uint64_t)h.draw_pos;  // item_env: the env's own global id unless a saved record was loaded
     if (p.item_mode == 0 && p.sample_dist) {  // C:bin3D.py:103-112
         auto u01 = [&](uint64_t salt) { return (double)(rnd_u64(p.seed ^ salt, gid, d) >> 11) * (1.0 / 9007199254740992.0); };
         auto r3 = [&](double v) { return ddiv(rint(v * 1000.0), 1000.0); };
@@ -139,7 +142,7 @@ __device__ __noinline__ void draw_item_c(const CParams &p, int e, CHdr &h) {
         h.next_den = p.setting == 3 ? rnd_density(p.seed, gid, d) : 1.0;
     } else {
         const double *it = p.item_mode == 0 ? p.item_set + (rnd_u64(p.seed, gid, d) % (uint64_t)p.n_items) * 3
-                                            : p.stream + ((size_t)e * p.stream_len + (size_t)(d % (uint64_t)p.stream_len)) * 4;
+                                            : p.stream + ((size_t)(h.item_env - p.env_id_base) * p.stream_len + (size_t)(d % (uint64_t)p.stream_len)) * 4;
         h.next_box[0] = it[0]; h.next_box[1] = it[1]; h.next_box[2] = it[2];
         h.next_den = p.setting == 3 ? (p.item_mode == 0 ? rnd_density(p.seed, gid, d) : it[3]) : 1.0;
     }
@@ -315,8 +318,9 @@ __global__ void __launch_bounds__(64) pctc_apply_kernel(const CParams p) {
     pct_step_info info{};
     if (p.mode == 0) {
         const int64_t dp = p.keep_draw ? h.draw_pos : 0;
+        const int64_t ie = p.keep_draw ? h.item_env : p.env_id_base + e;
         __syncwarp();
-        if (lane == 0) h.draw_pos = dp;
+        if (lane == 0) { h.draw_pos = dp; h.item_env = ie; }
         reset_space_c(ev, p, e, lane);
     } else {
         const double nb0 = h.next_box[0], nb1 = h.next_box[1], nb2 = h.next_box[2], den0 = h.next_den;
@@ -630,7 +634,7 @@ __global__ void __launch_bounds__(32) pctc_candidates_kernel(const CParams p) {
     __syncwarp();
     if (p.shuffle) {  // scratch: the GENEMS temp list (24 KB, idle between apply kernels): keys at 0, permuted codes at 10 KB
         static_assert(sizeof(ev->ems_tmp) >= 10240 + sizeof(ev->cand), "shuffle scratch fits");
-        shuffle_candidates<uint16_t>(ev->cand, cnt, (uint64_t *)ev->ems_tmp, (uint16_t *)((char *)ev->ems_tmp + 10240), p.seed, (uint64_t)(p.env_id_base + e),
+        shuffle_candidates<uint16_t>(ev->cand, cnt, (uint64_t *)ev->ems_tmp, (uint16_t *)((char *)ev->ems_tmp + 10240), p.seed, (uint64_t)h.item_env,
                                      (uint64_t)h.draw_pos, lane);
     }
     if (p.walkq) {
@@ -1117,6 +1121,117 @@ __global__ void pctc_policy_random_kernel(const CEnv *env, int n_envs, int64_t e
     leaf_idx[e] = n > 0 ? (int32_t)(rnd_u64(seed, (uint64_t)(env_id_base + e), (uint64_t)t) % (uint64_t)n) : 0;
 }
 
+// ================= saved env records (pct_save_envs / pct_load_envs) =================
+// Live between calls (cf. the discrete list next to DRec, pct_discrete.cu): the header, box / den [0, n_box), ems [0, n_ems), the load-edge
+// topology (e_off .. last_in, copied whole), e_st [0, n_edge), poly [0, n_poly), leaf [0, n_leaf), on ALIAS handles DEnvAux::box_st [0, n_box]
+// / e_upper [0, n_edge) / e_alias, and the LSAH footprint (4 doubles).  Not saved: ems_tmp (GENEMS / shuffle scratch), cand, big, fbits / n_fw
+// (per-step), lock / n_pending (zeroed on load).
+struct alignas(16) CRec {
+    RecHdr s;
+    CHdr h;
+    double box[NB_MAX][6];
+    double den[NB_MAX];
+    double ems[CE_MAX][6];
+    unsigned char topo[offsetof(CEnv, e_st) - offsetof(CEnv, e_off)];
+    Stack4 e_st[EDGE_MAX + 1];
+    double poly[POLY_MAX][2];
+    double leaf[NL_MAX][6];
+    Stack4 box_st[NB_MAX + 1];
+    uint8_t e_upper[EDGE_MAX + 1];
+    uint32_t e_alias[(EDGE_MAX + 32) / 32];
+    double hstate[4];
+};
+static_assert(sizeof(CHdr) % 16 == 0 && offsetof(CEnv, box) % 16 == 0 && offsetof(CEnv, den) % 16 == 0 && offsetof(CEnv, ems) % 16 == 0 &&
+              offsetof(CEnv, e_off) % 16 == 0 && offsetof(CEnv, e_st) % 16 == 0 && offsetof(CEnv, poly) % 16 == 0 && offsetof(CEnv, leaf) % 16 == 0,
+              "record parts are copied in 16-byte units");
+static_assert(offsetof(CRec, h) % 16 == 0 && offsetof(CRec, box) % 16 == 0 && offsetof(CRec, den) % 16 == 0 && offsetof(CRec, ems) % 16 == 0 &&
+              offsetof(CRec, topo) % 16 == 0 && offsetof(CRec, e_st) % 16 == 0 && offsetof(CRec, poly) % 16 == 0 && offsetof(CRec, leaf) % 16 == 0 &&
+              offsetof(CRec, box_st) % 16 == 0 && offsetof(CRec, e_upper) % 16 == 0 && offsetof(CRec, hstate) % 16 == 0, "record layout");
+
+// one warp per record; counts from the source's header, clamped to the capacities
+template <bool LOAD, typename OT>
+__global__ void __launch_bounds__(128, 4) pctc_env_record_kernel(const CParams p, const RecArgs s) {
+    const int lane = threadIdx.x & 31, i = blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (i >= s.n) return;
+    const int e = s.ids ? s.ids[i] : i;
+    CRec *r = (CRec *)(s.rec + (size_t)i * (size_t)s.rec_bytes);
+    if (e < 0 || e >= p.n_envs) {
+        if (LOAD) { if (lane == 0 && s.status) s.status[i] = REC_BAD_ENV; }
+        else if (lane == 0) { RecHdr z{}; z.magic = REC_MAGIC; z.version = REC_VERSION; r->s = z; }  // valid = 0
+        return;
+    }
+    CEnv *ev = p.env + e;
+    DEnvAux *aux = p.aux ? p.aux + e : nullptr;
+    const CHdr &src = LOAD ? r->h : ev->h;
+    if (LOAD) {
+        int st = 0;
+        if (lane == 0) st = rec_check(r->s, PCT_CONTINUOUS, src.item_env, s, p.env_id_base, p.n_envs);
+        st = __shfl_sync(FULL, st, 0);
+        if (lane == 0 && s.status) s.status[i] = st;
+        if (st) return;  // a rejected record leaves its env untouched
+    } else if (lane == 0) {
+        RecHdr z{};
+        z.magic = REC_MAGIC; z.version = REC_VERSION; z.domain = PCT_CONTINUOUS; z.valid = 1; z.fingerprint = s.fingerprint;
+        const int64_t row = src.item_env - p.env_id_base;
+        z.row_hash = (s.row_hash && row >= 0 && row < p.n_envs) ? s.row_hash[row] : 0;
+        r->s = z;
+    }
+    const int n_box = min(max(src.n_box, 0), NB_MAX), n_ems = min(max(src.n_ems, 0), CE_MAX), n_leaf = min(max(src.n_leaf, 0), NL_MAX);
+    const int n_edge = min(max(src.n_edge, 0), EDGE_MAX + 1), n_poly = min(max(src.n_poly, 0), POLY_MAX);
+    __syncwarp();
+    auto cp = [&](void *rec_part, void *env_part, int bytes) {
+        if (LOAD) warp_copy16(env_part, rec_part, bytes, lane);
+        else warp_copy16(rec_part, env_part, bytes, lane);
+    };
+    auto cp8 = [&](void *rec_part, void *env_part, int bytes) {
+        if (LOAD) warp_copy8(env_part, rec_part, bytes, lane);
+        else warp_copy8(rec_part, env_part, bytes, lane);
+    };
+    cp(&r->h, &ev->h, (int)sizeof(CHdr));
+    cp(r->box, ev->box, n_box * 48);
+    cp(r->den, ev->den, n_box * 8);
+    cp(r->ems, ev->ems, n_ems * 48);
+    cp(r->topo, ev->e_off, (int)sizeof(r->topo));
+    cp(r->e_st, ev->e_st, n_edge * (int)sizeof(Stack4));
+    cp(r->poly, ev->poly, n_poly * 16);
+    cp(r->leaf, ev->leaf, n_leaf * 48);
+    if (s.alias) {
+        cp8(r->box_st, aux->box_st, min(n_box + 1, NB_MAX + 1) * (int)sizeof(Stack4));
+        cp8(r->e_upper, aux->e_upper, n_edge);
+        if (lane < (EDGE_MAX + 32) / 32) { if (LOAD) aux->e_alias[lane] = r->e_alias[lane]; else r->e_alias[lane] = aux->e_alias[lane]; }
+    }
+    if (lane < 2) {
+        uint4 *hs = (uint4 *)((double *)s.hstate + (size_t)e * 4) + lane;
+        if (LOAD) *hs = ((const uint4 *)r->hstate)[lane]; else ((uint4 *)r->hstate)[lane] = *hs;
+    }
+    if (LOAD) {
+        if (lane == 0) { ev->lock = 0; ev->n_pending = 0; }
+        if (aux && lane == 0) { aux->obs_prev[0] = p.nb; aux->obs_prev[1] = p.nl; }  // the next step rewrites every row of whichever buffer it gets
+        if (p.obs) {
+            __syncwarp();
+            write_obs_c<OT>(p, e, ev, ev->leaf, n_leaf, lane, 32);
+        }
+    }
+}
+
+int64_t continuous_record_bytes() { return (int64_t)sizeof(CRec); }
+
+// plain stream-ordered launches, see launch_records_discrete
+int continuous_records(pct_env_batch *h, const RecArgs &s, int load, void *obs, cudaStream_t st) {
+    if (s.n <= 0) return PCT_OK;
+    CParams p{};
+    p.env = (CEnv *)h->c_state; p.n_envs = h->n_envs;
+    p.H = h->cfg.container_size[2]; p.nb = h->cfg.internal_node_holder; p.nl = h->cfg.leaf_node_holder;
+    p.env_id_base = h->cfg.env_id_base; p.aux = h->d_aux; p.obs = obs;
+    const int blocks = (s.n + 3) / 4;
+    if (!load) pctc_env_record_kernel<false, float><<<blocks, 128, 0, st>>>(p, s);
+    else if (h->cfg.obs_dtype == PCT_F64) pctc_env_record_kernel<true, double><<<blocks, 128, 0, st>>>(p, s);
+    else pctc_env_record_kernel<true, float><<<blocks, 128, 0, st>>>(p, s);
+    const cudaError_t e = cudaGetLastError();
+    if (e != cudaSuccess) { h->err = std::string("env records: ") + cudaGetErrorString(e); return PCT_ERR_CUDA; }
+    return PCT_OK;
+}
+
 // ================= host side =================
 int continuous_create(pct_env_batch *h) {
     cudaError_t e = cudaMalloc(&h->c_state, sizeof(CEnv) * (size_t)h->n_envs);
@@ -1132,6 +1247,12 @@ int continuous_create(pct_env_batch *h) {
         if (e == cudaSuccess && h->walk_fork) e = cudaMalloc(&h->d_walk_pend, sizeof(int32_t) * (size_t)CAND_MAX * (size_t)h->n_envs);
         h->contq_env_bytes = h->walk_fork ? sizeof(WalkPiece) * (size_t)WALK_PIECES_PER_ENV : sizeof(WalkCont) * (size_t)WALK_CONT_PER_ENV;
         if (e == cudaSuccess) e = cudaMalloc((void **)&h->d_contq, h->contq_env_bytes * (size_t)h->n_envs);
+    }
+    if (e == cudaSuccess) {  // item_env = the env's own global id (CHdr::item_env)
+        std::vector<int64_t> id((size_t)h->n_envs);
+        for (int i = 0; i < h->n_envs; i++) id[i] = h->cfg.env_id_base + i;
+        e = cudaMemcpy2D((char *)h->c_state + offsetof(CEnv, h) + offsetof(CHdr, item_env), sizeof(CEnv), id.data(), sizeof(int64_t), sizeof(int64_t),
+                         (size_t)h->n_envs, cudaMemcpyHostToDevice);
     }
     if (e != cudaSuccess) { h->err = std::string("continuous_create: ") + cudaGetErrorString(e); return PCT_ERR_CUDA; }
     return PCT_OK;

@@ -27,6 +27,7 @@
 #include "pct_kernels.h"
 #include "pct_geom.cuh"
 #include "pct_walkq.cuh"
+#include "pct_records.cuh"
 
 namespace pct {
 
@@ -541,14 +542,14 @@ __device__ __noinline__ int gen_level_points(const int16_t (*box)[6], int n_box,
 
 // ---- item source ------------------------------------------------------------------------------------------
 __device__ __noinline__ void draw_item(const DParams &p, int e, DHdr &h) {
-    const uint64_t gid = (uint64_t)(p.env_id_base + e);
+    const uint64_t gid = (uint64_t)h.item_env;  // the env's own global id unless a saved record was loaded into it
     const uint64_t d = (uint64_t)h.draw_pos;
     const double *it;
     if (p.item_mode == 0) {
         it = p.item_set + (rnd_u64(p.seed, gid, d) % (uint64_t)p.n_items) * 3;
         h.next_den = p.setting == 3 ? rnd_density(p.seed, gid, d) : 1.0;
     } else {
-        it = p.stream + ((size_t)e * p.stream_len + (size_t)(d % (uint64_t)p.stream_len)) * 4;
+        it = p.stream + ((size_t)(h.item_env - p.env_id_base) * p.stream_len + (size_t)(d % (uint64_t)p.stream_len)) * 4;
         h.next_den = p.setting == 3 ? it[3] : 1.0;
     }
     h.next_box[0] = (int)it[0];
@@ -767,9 +768,10 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK, K1_MINB) pct_apply_kerne
     if (p.mode == 0) {
         // ---------------- reset (D:bin3D.py:61-67, D:space.py:290-314) ----------------
         const int64_t dp = p.keep_draw ? ghot->h.draw_pos : 0;  // box_creator.reset() does not rewind the item source
+        const int64_t ie = p.keep_draw ? ghot->h.item_env : p.env_id_base + e;  // ... nor change the sequence it follows
         for (int t = lane; t < (int)(sizeof(DEnvHot) / 4); t += 32) ((uint32_t *)hot)[t] = 0;
         __syncwarp();
-        if (lane == 0) hot->h.draw_pos = dp;
+        if (lane == 0) { hot->h.draw_pos = dp; hot->h.item_env = ie; }
         __syncwarp();
         reset_space(hot, p, e, lane);
     } else {
@@ -1020,7 +1022,7 @@ __global__ void __launch_bounds__(32 * WARPS_PER_BLOCK) pct_candidates_kernel(co
     if (p.shuffle) {  // scratch: cold->raw + cold->tab_big (contiguous, 16 KB, free once the list is in `out`): keys at 0, permuted list at 10 KB
         static_assert(offsetof(DEnvCold, tab_big) == offsetof(DEnvCold, raw) + sizeof(uint32_t) * RAW_MAX, "raw and tab_big are contiguous");
         static_assert(CAND_MAX * 8 <= 10240 && 10240 + CAND_MAX * 4 <= (RAW_MAX + TAB_A) * 4, "shuffle scratch fits");
-        shuffle_candidates<SlotT>(out, n_cand, (uint64_t *)cold->raw, (SlotT *)((char *)cold->raw + 10240), p.seed, (uint64_t)(p.env_id_base + e),
+        shuffle_candidates<SlotT>(out, n_cand, (uint64_t *)cold->raw, (SlotT *)((char *)cold->raw + 10240), p.seed, (uint64_t)h.item_env,
                                   (uint64_t)h.draw_pos, lane);
         cand = out;
     }
@@ -1546,6 +1548,116 @@ __global__ void pct_fill_prev_kernel(DEnvAux *aux, int n, int nb, int nl) {
 }
 void launch_fill_prev(DEnvAux *aux, int n_envs, int nb, int nl, cudaStream_t st) {
     pct_fill_prev_kernel<<<(n_envs + 255) / 256, 256, 0, st>>>(aux, n_envs, nb, nl);
+}
+
+// ---- saved env records (pct_save_envs / pct_load_envs) ------------------------------------------------------------------------------------
+// What stays live between two calls, read off the kernels above (everything else is per-step scratch, rebuilt by the next step before it is read):
+//   DEnvHot              whole (3.5 KB): header (counts, item source position + item_env, episode sums, flags, next item), boxes, EMS list,
+//                        load-edge topology (e_off / e_lower / e_next / first_in / last_in / poly_off)
+//   DEnvCold::leaf       [0, n_leaf)   leaves of the last observation (leaf-index actions, observation on load)
+//   DEnvCold::density    [0, n_box)    per placed box (setting 3)
+//   DEnvCold::e_st       [0, n_edge)   loads of the edge pool (stability settings)
+//   DEnvCold::poly       [0, n_poly)   support-polygon vertices
+//   DEnvAux::box_st      [0, n_box]    ALIAS handles only (PCT_B200_ALIAS=0 handles never write it); entry n_box is the stack of the last placement
+//                                      attempt, rewritten by the next one before it is read — saved anyway, it costs 32 bytes
+//   DEnvAux::e_upper     [0, n_edge), DEnvAux::e_alias (32 bytes)   ALIAS handles only
+//   LSAH footprint       4 int32 (pct_heuristic_actions)
+// Not saved: cand / raw / tab_big (written by K2 before K3 / emit read them), fbits / n_fw (written by K2's classification, read by the walk
+// and emit kernels of the same step), big (per-descent scratch), lock / n_pending (zeroed on load; both are zero between calls), obs_prev
+// (set to "every row" on load).  No kernel reads an array beyond its count: after an auto-reset every array still holds the previous episode.
+struct alignas(16) DRec {
+    RecHdr s;
+    DEnvHot hot;
+    int16_t leaf[NL_MAX][6];
+    double density[NB_MAX];
+    Stack4 e_st[EDGE_MAX + 1];
+    double poly[POLY_MAX][2];
+    Stack4 box_st[NB_MAX + 1];
+    uint8_t e_upper[EDGE_MAX + 1];
+    uint32_t e_alias[(EDGE_MAX + 32) / 32];
+    int32_t hstate[4];
+};
+static_assert(offsetof(DEnvCold, leaf) % 16 == 0 && offsetof(DEnvCold, density) % 16 == 0 && offsetof(DEnvCold, e_st) % 16 == 0 &&
+              offsetof(DEnvCold, poly) % 16 == 0 && sizeof(DEnvCold) % 16 == 0, "cold arrays are copied in 16-byte units");
+static_assert(offsetof(DEnvAux, e_upper) % 8 == 0 && sizeof(DEnvAux) % 8 == 0 && sizeof(DEnvAux::e_alias) == 32, "aux arrays are copied in 8-byte units");
+static_assert(offsetof(DRec, leaf) % 16 == 0 && offsetof(DRec, density) % 16 == 0 && offsetof(DRec, e_st) % 16 == 0 && offsetof(DRec, poly) % 16 == 0 &&
+              offsetof(DRec, box_st) % 16 == 0 && offsetof(DRec, e_upper) % 16 == 0 && offsetof(DRec, hstate) % 16 == 0, "record layout");
+int64_t discrete_record_bytes() { return (int64_t)sizeof(DRec); }
+
+// One warp per record.  Counts come from the source's header (clamped to the capacities).
+template <bool LOAD, typename OT>
+__global__ void __launch_bounds__(128, 4) pct_env_record_kernel(const DParams p, const RecArgs s) {
+    const int lane = threadIdx.x & 31, i = blockIdx.x * 4 + (threadIdx.x >> 5);
+    if (i >= s.n) return;
+    const int e = s.ids ? s.ids[i] : i;
+    DRec *r = (DRec *)(s.rec + (size_t)i * (size_t)s.rec_bytes);
+    if (e < 0 || e >= p.n_envs) {
+        if (LOAD) { if (lane == 0 && s.status) s.status[i] = REC_BAD_ENV; }
+        else if (lane == 0) { RecHdr z{}; z.magic = REC_MAGIC; z.version = REC_VERSION; r->s = z; }  // valid = 0
+        return;
+    }
+    DEnvHot *hot = p.hot + e;
+    DEnvCold *cold = p.cold + e;
+    DEnvAux *aux = p.aux ? p.aux + e : nullptr;
+    const DHdr &src = LOAD ? r->hot.h : hot->h;
+    if (LOAD) {
+        int st = 0;
+        if (lane == 0) st = rec_check(r->s, PCT_DISCRETE, src.item_env, s, p.env_id_base, p.n_envs);
+        st = __shfl_sync(FULL, st, 0);
+        if (lane == 0 && s.status) s.status[i] = st;
+        if (st) return;  // a rejected record leaves its env untouched
+    } else if (lane == 0) {
+        RecHdr z{};
+        z.magic = REC_MAGIC; z.version = REC_VERSION; z.domain = PCT_DISCRETE; z.valid = 1; z.fingerprint = s.fingerprint;
+        const int64_t row = src.item_env - p.env_id_base;
+        z.row_hash = (s.row_hash && row >= 0 && row < p.n_envs) ? s.row_hash[row] : 0;
+        r->s = z;
+    }
+    const int n_box = min(max(src.n_box, 0), NB_MAX), n_leaf = min(max(src.n_leaf, 0), NL_MAX);
+    const int n_edge = min(max(src.n_edge, 0), EDGE_MAX + 1), n_poly = min(max(src.n_poly, 0), POLY_MAX);
+    __syncwarp();
+    auto cp = [&](void *rec_part, void *env_part, int bytes) {
+        if (LOAD) warp_copy16(env_part, rec_part, bytes, lane);
+        else warp_copy16(rec_part, env_part, bytes, lane);
+    };
+    auto cp8 = [&](void *rec_part, void *env_part, int bytes) {
+        if (LOAD) warp_copy8(env_part, rec_part, bytes, lane);
+        else warp_copy8(rec_part, env_part, bytes, lane);
+    };
+    cp(&r->hot, hot, (int)sizeof(DEnvHot));
+    cp(r->leaf, cold->leaf, n_leaf * 12);
+    cp(r->density, cold->density, n_box * 8);
+    cp(r->e_st, cold->e_st, n_edge * (int)sizeof(Stack4));
+    cp(r->poly, cold->poly, n_poly * 16);
+    if (s.alias) {
+        cp8(r->box_st, aux->box_st, min(n_box + 1, NB_MAX + 1) * (int)sizeof(Stack4));
+        cp8(r->e_upper, aux->e_upper, n_edge);
+        if (lane < (EDGE_MAX + 32) / 32) { if (LOAD) aux->e_alias[lane] = r->e_alias[lane]; else r->e_alias[lane] = aux->e_alias[lane]; }
+    }
+    if (lane == 0) {
+        uint4 *hs = (uint4 *)((int32_t *)s.hstate + (size_t)e * 4);
+        if (LOAD) *hs = *(const uint4 *)r->hstate; else *(uint4 *)r->hstate = *hs;
+    }
+    if (LOAD) {
+        if (lane == 0) { cold->lock = 0; cold->n_pending = 0; }
+        if (aux && lane == 0) { aux->obs_prev[0] = p.nb; aux->obs_prev[1] = p.nl; }  // the next step rewrites every row of whichever buffer it gets
+        if (p.obs) {
+            __syncwarp();  // the warp's copies above are visible to all its lanes
+            write_obs<OT, 0>(p, e, hot, cold, cold->leaf, n_leaf, lane, 32);
+        }
+    }
+}
+
+// Plain stream-ordered launches (no programmatic serialisation): a save / load sits between the previous step's emit kernel and the next
+// step's apply kernel.  The LPT bucket lists (order_file / order_lookup) stay a permutation of the envs after a load, so they need no update;
+// d_ready / epoch belong to the step's kernels and are not touched.
+cudaError_t launch_records_discrete(const DParams &p, const RecArgs &s, int load, cudaStream_t st) {
+    if (s.n <= 0) return cudaSuccess;
+    const int blocks = (s.n + 3) / 4;
+    if (!load) pct_env_record_kernel<false, float><<<blocks, 128, 0, st>>>(p, s);
+    else if (p.obs_f64) pct_env_record_kernel<true, double><<<blocks, 128, 0, st>>>(p, s);
+    else pct_env_record_kernel<true, float><<<blocks, 128, 0, st>>>(p, s);
+    return cudaGetLastError();
 }
 
 // ---- launchers ---------------------------------------------------------------------------------------------

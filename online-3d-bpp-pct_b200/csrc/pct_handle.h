@@ -20,6 +20,8 @@ struct pct_env_batch {
     int n_items = 0;
     double *d_stream = nullptr;
     int stream_len = 0;
+    uint64_t item_set_hash = 0;   // content hash of the item set (part of the record fingerprint, pct_api.cu config_fingerprint)
+    uint64_t *d_row_hash = nullptr;  // [n_envs] content hash of every item-stream row: a loaded record must find the row it draws from unchanged
     int traj_len = 0;
     int32_t *d_ready = nullptr;   // [2 * n_envs] per-env hand-over flags of the overlapped launch mode
     int32_t epoch = 0;
@@ -41,7 +43,7 @@ struct pct_env_batch {
     bool fill_pending = false;
     bool host_zero_copy = true;   // pct_step_host: kernels write the observation straight into the pinned (mapped) host buffer; PCT_B200_HOST_ZEROCOPY=0: staged copies
     bool cont_pre = true;         // continuous feas_emit: resting heights from pre-rounded rectangles (exact, +2 %; PCT_B200_CONT_PRE=0 disables)
-    int32_t *d_hstate = nullptr;  // (n_envs, 4) LSAH footprint state (pct_heuristic_actions)
+    int32_t *d_hstate = nullptr;  // (n_envs, 4) LSAH footprint state (pct_heuristic_actions); allocated at pct_create (per-env state: saved records carry it)
     double *d_hstate_c = nullptr; // same for the continuous domain (pct_heuristic_actions_f64)
     double *d_query_c = nullptr;  // 2 doubles: result of pct_query_placement_f64
     int32_t *d_query = nullptr;   // 2 + W*L ints: result of pct_query_placement

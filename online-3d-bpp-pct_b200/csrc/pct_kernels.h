@@ -1,5 +1,6 @@
 // Internal: device record layouts and kernel launch parameters shared by the kernels and the C-ABI layer.
 #pragma once
+#include <cstddef>
 #include <cstdint>
 #include <cuda_runtime.h>
 #include "pct_b200.h"
@@ -109,6 +110,7 @@ struct alignas(16) DHdr {  // 64 bytes
     int32_t ep_len;
     int32_t n_cand;
     int32_t n_poly;        // vertices in the polygon pool
+    int64_t item_env;      // global env id whose item sequence this env follows (its own id unless a saved record was loaded into it)
 };
 struct alignas(16) DEnvHot {
     DHdr h;
@@ -124,6 +126,7 @@ struct alignas(16) DEnvHot {
 constexpr int HOT_PREFIX = sizeof(DHdr) + NB_MAX * 12 + E_MAX * 12;
 static_assert(HOT_PREFIX % 16 == 0, "prefix is a TMA bulk copy");
 static_assert(sizeof(DHdr) == 72 || sizeof(DHdr) == 80 || sizeof(DHdr) == 64, "header size");
+static_assert(offsetof(DHdr, item_env) == 72 && sizeof(DHdr) == 80, "item_env sits in the header's former padding");
 static_assert(sizeof(DEnvHot) % 16 == 0, "TMA bulk copies move multiples of 16 bytes");
 
 // "Cold" record: touched only by the paths that need it (leaf-index actions, setting-3 densities, the
@@ -262,5 +265,32 @@ int discrete_kernels_per_step(const DParams &p);
 cudaError_t launch_discrete(const DParams &p, cudaStream_t st, cudaEvent_t *prof = nullptr);
 cudaError_t launch_policy_random_discrete(const DEnvHot *hot, int n_envs, int64_t env_id_base, uint64_t seed, int64_t t, int32_t *leaf_idx,
                                           cudaStream_t st, const int64_t *t_dev = nullptr);
+
+// ---- saved env records (pct_save_envs / pct_load_envs) -------------------------------------------------------
+// A record is a fixed-size, 16-byte-aligned slot: this header, then the domain's layout (DRec in pct_discrete.cu, CRec in pct_continuous.cu).
+constexpr uint32_t REC_MAGIC = 0x52544350u;  // "PCTR"
+constexpr uint32_t REC_VERSION = 1;
+constexpr int REC_BAD_RECORD = 1, REC_ROW_OUTSIDE = 2, REC_BAD_ENV = 3;  // pct_load_envs status codes (0 = loaded)
+struct alignas(16) RecHdr {
+    uint32_t magic, version, domain, valid;  // valid = 0: written for an env id outside the saving handle
+    uint64_t fingerprint;  // configuration fingerprint of the saving handle (pct_api.cu, config_fingerprint)
+    uint64_t row_hash;     // item-stream mode: content hash of the stream row the env draws from (its item_env); 0 otherwise
+    uint64_t pad_[4];
+};
+static_assert(sizeof(RecHdr) == 64, "record header");
+struct RecArgs {
+    const int32_t *ids;       // [n] env ids (nullptr: record i <-> env i)
+    int n;
+    unsigned char *rec;       // n records of rec_bytes each (read-only for a load)
+    int64_t rec_bytes;
+    uint64_t fingerprint;
+    const uint64_t *row_hash; // item-stream mode: content hash of every stream row of this handle [n_envs]; nullptr otherwise
+    int alias;                // DEnvAux::box_st / e_upper / e_alias are live (ALIAS apply kernels)
+    void *hstate;             // LSAH footprint, 4 words per env (int32 discrete, double continuous)
+    int32_t *status;          // load: [n] per-record codes, may be nullptr
+};
+int64_t discrete_record_bytes();
+// save (load == 0) or load (load == 1) of the records in `s`; p: state_params of the handle + obs / obs_f64 / aux
+cudaError_t launch_records_discrete(const DParams &p, const RecArgs &s, int load, cudaStream_t st);
 
 }  // namespace pct

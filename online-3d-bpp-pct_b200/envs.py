@@ -9,6 +9,8 @@ observations as the reference returns them), so `evaluation_tools.evaluate` (eva
 heuristics' read-only attribute accesses work unchanged.  They exist for drop-in compatibility; throughput comes
 from PctVecEnv / PctBatch.
 """
+import copy
+
 import numpy as np
 import torch
 
@@ -71,6 +73,11 @@ class _PackingBase(object):
                  item_stream=None, size_minimum=None, **kwags):
         if next_holder != 1:
             raise NotImplementedError("next_holder must be 1 (reference default)")
+        self._init_args = (setting, dict(container_size=container_size, item_set=item_set, data_name=data_name, load_test_data=load_test_data,
+                                         internal_node_holder=internal_node_holder, leaf_node_holder=leaf_node_holder, next_holder=next_holder,
+                                         shuffle=shuffle, LNES=LNES, sample_from_distribution=sample_from_distribution,
+                                         sample_left_bound=sample_left_bound, sample_right_bound=sample_right_bound, device=device, seed=seed,
+                                         item_stream=item_stream, size_minimum=size_minimum, **kwags))  # __deepcopy__ builds its twin from them
         self.internal_node_holder, self.leaf_node_holder, self.next_holder = internal_node_holder, leaf_node_holder, next_holder
         self.bin_size = container_size
         self.setting = setting
@@ -137,6 +144,20 @@ class _PackingBase(object):
 
     def close(self):
         self._batch.close()
+
+    def __deepcopy__(self, memo):
+        """copy.deepcopy(env), as search / lookahead code does with the reference's plain-Python env: an independent env in the same state that
+        continues exactly like this one under the same actions (a new batch of one with the same constructor arguments, reset, then loaded with
+        this env's saved record).  The items drawn after the copy are the original's too (DESIGN.md 3(d): the copy follows the original's item
+        sequence); with RandomBoxCreator the reference's copies share numpy's global RNG instead and do not replay."""
+        setting, kw = self._init_args
+        new = type(self).__new__(type(self))
+        memo[id(self)] = new
+        _PackingBase.__init__(new, setting, **kw)
+        new._batch.reset()
+        new._batch.load_envs(self._batch.save_envs())
+        new._next_box_override = copy.deepcopy(self._next_box_override, memo)
+        return new
 
     @property
     def unwrapped(self):
